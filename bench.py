@@ -10,6 +10,8 @@ GPU, bf16).
     python bench.py --global-batch 16 ...       # strong scaling: the global batch is fixed and sharded over the ranks
     python bench.py --sweep                     # every BASELINE config + the keypoint batch sweep, one JSON line each
     python bench.py --impl reference ...        # the reference's own PLMSSampler + UNetModel on the host cores
+    python bench.py --dump-outputs DIR ...      # also write the last timed step's final latent(s) to DIR/*.npy
+    python bench.py --per-op-json FILE ...      # also write the kernel pass's per-op times to FILE
 
 One "step" = one full `PLMSSampler.sample(S=50)` of one batch = 102 UNet forwards per image (cond + uncond
 x (50 + 1)); weights are seeded random of the SD-1.4 + GLIGEN architecture (no checkpoints offline), inputs
@@ -37,6 +39,7 @@ from gligen_b200 import synth  # noqa: E402
 from gligen_b200.spec import NAMED_CONFIGS, flops_per_forward, synthetic_state_dict  # noqa: E402
 
 UNIT = "images/s"
+DUMP_BYTES = 64 * 10 ** 6          # --dump-outputs: bound on the arrays of all ranks together
 # BASELINE.json configs[1..4] (configs[0] is the reference's CPU plumbing case: a parity test, not a bench line)
 PRESETS = {
     2: dict(config="sd14_box_text", batch=4, alpha_type="1,0,0", what="box+text"),
@@ -64,6 +67,10 @@ def parse(argv=None):
     ap.add_argument("--no-kernel-pass", action="store_true")
     ap.add_argument("--sweep", action="store_true", help="all BASELINE configs + keypoint batch sweep (1 GPU); one JSON line each")
     ap.add_argument("--ref-budget-s", type=float, default=200.0, help="reference arm: wall-clock budget that sizes its bounded sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the final latent of the last timed step as DIR/<name>.npy (float32)")
+    ap.add_argument("--per-op-json", metavar="FILE", default=None,
+                    help="write the kernel pass's per-op GPU times, flops and bytes to FILE (scripts/summarize_profiles.py reads them)")
     args = ap.parse_args(argv)
     if args.preset:
         pr = PRESETS[args.preset]
@@ -395,12 +402,14 @@ def run_ours(args, world, rank, local_rank, dev, quiet_extras=False):
             torch.distributed.barrier()
         torch.cuda.synchronize()
 
+    last = [None]
+
     def timed(n, from_host):
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(n):
-            one_image_batch(from_host)
+            last[0] = one_image_batch(from_host)
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -416,12 +425,16 @@ def run_ours(args, world, rank, local_rank, dev, quiet_extras=False):
     _quiet.__enter__()
     for _ in range(args.warmup):
         one_image_batch(False)
+    # the inpainting sampler draws q_sample noise from the global generator: a fixed seed here makes the timed steps'
+    # inputs identical from run to run, whatever the code before this point drew
+    torch.manual_seed(1234)
     clocks = ClockSampler(local_rank)
     clocks.start()
     l0 = eng.kernel_launches
     ms = timed(args.steps, False)
     launches = eng.kernel_launches - l0 + (args.steps * (S + 1) if B else 0)          # + the fused sampler-update kernels
     clk = clocks.stop()
+    final_latent = last[0].float().cpu() if last[0] is not None else None
     one_image_batch(True)
     ms_e2e = timed(args.steps, True)
     _quiet.__exit__(None, None, None)
@@ -459,9 +472,9 @@ def run_ours(args, world, rank, local_rank, dev, quiet_extras=False):
                          "achieved": tc_fl / (tc_ms * 1e-3) / 1e12, "frac": tc_fl / (tc_ms * 1e-3) / 1e12 / peak_tf,
                          "flops_per_launch": tc_fl / max(tc_n, 1), "avg_launch_ms": tc_ms / max(tc_n, 1), "launches_per_forward": tc_n,
                          "forward_ms_sum_of_ops": tot_ms, "op_timing": "each op replayed from its own CUDA graph (GPU time, no host issue time)"})
-            if not quiet_extras:
-                os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-                with open(os.path.join(ROOT, "gpurun_out", "bench_per_op.json"), "w") as f:
+            if args.per_op_json and not quiet_extras:
+                os.makedirs(os.path.dirname(args.per_op_json), exist_ok=True)
+                with open(args.per_op_json, "w") as f:
                     json.dump([dict(name=n, kind=k, gflop=fl / 1e9, mbytes=by / 1e6, ms=m) for n, k, fl, by, m in per_op], f)
         for tname in ("r2_gemm_dram_traffic.json", "r1_gemm_dram_traffic.json"):
             tpath = os.path.join(ROOT, "profiles", tname)
@@ -490,16 +503,34 @@ def run_ours(args, world, rank, local_rank, dev, quiet_extras=False):
                 "gpu_launches": int(launches), "clocks": clk, "roofline": roof, "cpu_baseline": cpu, "kernel_shares": kernel_shares}
     del sampler, model, eng
     torch.cuda.empty_cache()
-    return line
+    return line, final_latent
+
+
+def dump_outputs(dirname, arrays, budget):
+    """Write each tensor of `arrays` as dirname/<name>.npy in float32.  When they hold more than `budget` bytes in all,
+    each is replaced by the same fraction of its elements, flattened, at indices drawn from a fixed seed."""
+    os.makedirs(dirname, exist_ok=True)
+    total = 4 * sum(t.numel() for t in arrays.values())
+    for name, t in arrays.items():
+        a = t.float().cpu().numpy()
+        if total > budget:
+            keep = a.size * budget // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def main():
     args = parse()
+    if args.impl == "reference" and args.dump_outputs:
+        raise SystemExit("--dump-outputs writes what the timed GPU path computed: it needs --impl ours")
     if args.impl == "reference":
         line = run_reference(args)
         if line is not None:
             print(json.dumps(line))
         return
+    for k in ("dump_outputs", "per_op_json"):                        # run_ours changes the working directory
+        if getattr(args, k):
+            setattr(args, k, os.path.abspath(getattr(args, k)))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -512,25 +543,33 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     assert world == args.gpus, f"--gpus {args.gpus} but WORLD_SIZE={world} (launch with torch.distributed.run)"
     cwd = os.getcwd()
+    suffix = f"_rank{rank}" if world > 1 else ""
+    outputs = {}
     if args.sweep:
         # every BASELINE.json config at its own batch + the keypoint batch sweep (config 5), short runs; one line each
         cases = [dict(preset=2), dict(preset=2, alpha_type="0.3,0,0.7"), dict(preset=3), dict(preset=4)]
         cases += [dict(preset=5, batch=b) for b in (1, 2, 4, 8, 16, 32, 64)]
-        for c in cases:
+        for i, c in enumerate(cases):
             a = parse(["--preset", str(c["preset"]), "--steps", str(args.steps), "--warmup", str(args.warmup), "--gpus", str(args.gpus)] +
                       (["--batch", str(c["batch"])] if "batch" in c else []) + (["--alpha-type", c["alpha_type"]] if "alpha_type" in c else []))
             if "batch" in c:
                 a.batch = c["batch"]
             a.no_kernel_pass = args.no_kernel_pass
             os.chdir(cwd)
-            line = run_ours(a, world, rank, local_rank, dev, quiet_extras=True)
+            line, lat = run_ours(a, world, rank, local_rank, dev, quiet_extras=True)
+            if lat is not None:
+                outputs[f"sweep{i:02d}_latent{suffix}"] = lat
             if line is not None:
                 line["sweep"] = True
                 print(json.dumps(line), flush=True)
     else:
-        line = run_ours(args, world, rank, local_rank, dev)
+        line, lat = run_ours(args, world, rank, local_rank, dev)
+        if lat is not None:
+            outputs["latent" + suffix] = lat
         if line is not None:
             print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs, DUMP_BYTES // world)
     if world > 1:
         torch.distributed.destroy_process_group()
 

@@ -14,6 +14,7 @@ For each configuration it
 from __future__ import annotations
 
 import argparse
+import hashlib
 import os
 import sys
 import time
@@ -271,7 +272,7 @@ def scalar_anchors():
     print("anchors:", te[0, :2].tolist(), fe[0, :4].tolist(), float(sched["alphas_cumprod"][0]), float(al[0]), float(al[-1]), float(alp[-1]))
 
 
-def run_vae(name, B, seed=3, store_half=False):
+def run_vae(name, B, seed=3, store_half=False, image_stride=1):
     """SURVEY 8(f) rank 1 (next row): pin oracle/vae_oracle.py against the reference AutoencoderKL.decode."""
     from gligen_b200.spec import NAMED_VAE_CONFIGS, synthetic_vae_state_dict, vae_decoder_param_shapes
     from oracle import vae_oracle as VO
@@ -298,11 +299,13 @@ def run_vae(name, B, seed=3, store_half=False):
     diff = (img - mine_img).abs().max().item()
     print(f"{name}: reference decode {tuple(img.shape)} in {t_ref:.1f} s; max |oracle - reference| = {diff:.3e}; mean |img| = {img.abs().mean():.3f}")
     assert diff <= 1e-4 * max(1.0, img.abs().max().item())
-    torch.save({"name": name, "B": B, "seed": seed, "z": z, "image": img.half() if store_half else img, "oracle_max_abs_diff": diff},
+    img = img[..., ::image_stride, ::image_stride]          # every image_stride-th row and column: keeps the fixture under 1 MB
+    torch.save({"name": name, "B": B, "seed": seed, "z": z, "image": img.half() if store_half else img, "image_stride": image_stride,
+                "oracle_max_abs_diff": diff},
                os.path.join(GOLD, f"{name}_B{B}.pt"))
 
 
-def run_vae_encode(name, B, seed=5, store_half=False):
+def run_vae_encode(name, B, seed=5, store_half=False, x_from_seed=False):
     """SURVEY 8(f) rank 3 (encoder half): pin oracle/vae_oracle.vae_encode_moments / vae_encode against the reference
     AutoencoderKL.encode (same synthetic weights, same image, same global CPU seed for the posterior noise)."""
     from gligen_b200.spec import NAMED_VAE_CONFIGS, synthetic_vae_encoder_state_dict, vae_encoder_param_shapes
@@ -319,12 +322,7 @@ def run_vae_encode(name, B, seed=5, store_half=False):
     sd = synthetic_vae_encoder_state_dict(cfg, 1)
     missing, unexpected = ref.load_state_dict(sd, strict=False)
     assert not unexpected and all(k.startswith(("decoder.", "post_quant_conv.")) for k in missing)
-    g = torch.Generator().manual_seed(seed)
-    S = cfg.image_size
-    # a smooth image in [-1, 1] plus texture (what `encode` sees: a normalised RGB picture)
-    yy, xx = torch.meshgrid(torch.linspace(-1, 1, S), torch.linspace(-1, 1, S), indexing="ij")
-    base = torch.stack([torch.sin(3 * xx + c) * torch.cos(2 * yy - c) for c in range(cfg.in_channels)], 0)
-    x = (0.7 * base[None] + 0.3 * torch.randn(B, cfg.in_channels, S, S, generator=g)).clamp(-1, 1)
+    x = VO.encode_test_image(cfg, B, seed)
     if store_half:
         x = x.half().float()               # the fixture stores the image as fp16: run the reference on exactly those values
     t0 = time.time()
@@ -341,9 +339,12 @@ def run_vae_encode(name, B, seed=5, store_half=False):
     print(f"{name}: reference encode {tuple(x.shape)} -> {tuple(mom.shape)} in {t_ref:.1f} s; max |oracle - reference| moments {diff:.3e}, "
           f"sample {diff_z:.3e}; mean |mean| {mom[:, :cfg.embed_dim].abs().mean():.3f}, logvar range [{mom[:, cfg.embed_dim:].min():.2f}, {mom[:, cfg.embed_dim:].max():.2f}]")
     assert diff <= 1e-4 * max(1.0, mom.abs().max().item()) and diff_z <= 1e-4 * max(1.0, z0.abs().max().item())
-    torch.save({"name": name, "B": B, "seed": seed, "noise_seed": 1234, "x": x.half() if store_half else x, "moments": mom, "z0": z0,
-                "oracle_max_abs_diff": diff},
-               os.path.join(GOLD, f"{name}_enc_B{B}.pt"))
+    out = {"name": name, "B": B, "seed": seed, "noise_seed": 1234, "moments": mom, "z0": z0, "oracle_max_abs_diff": diff}
+    if x_from_seed:             # keeps the fixture under 1 MB: tests rebuild x with VO.encode_test_image and check the hash
+        out["x_sha256"] = hashlib.sha256(x.half().numpy().tobytes()).hexdigest()
+    else:
+        out["x"] = x.half() if store_half else x
+    torch.save(out, os.path.join(GOLD, f"{name}_enc_B{B}.pt"))
 
 
 if __name__ == "__main__":
@@ -361,13 +362,13 @@ if __name__ == "__main__":
         run_vae("tiny_vae", B=2)
         run_vae("tiny_vae64", B=2)
         run_vae("small_vae", B=1, store_half=True)
-        run_vae("sd14_vae", B=1, store_half=True)
+        run_vae("sd14_vae", B=1, store_half=True, image_stride=2)
         sys.exit(0)
     if args.vae_enc:
         run_vae_encode("tiny_vae", B=2)
         run_vae_encode("tiny_vae64", B=2)
         run_vae_encode("small_vae", B=1, store_half=True)
-        run_vae_encode("sd14_vae", B=1, store_half=True)
+        run_vae_encode("sd14_vae", B=1, store_half=True, x_from_seed=True)
         sys.exit(0)
     if args.configs345:
         # BASELINE config 3 (box + text + image: 30 objects -> 60 grounding tokens), config 5 (keypoint: 8 x 17 = 136

@@ -58,6 +58,16 @@ def attn_block(x, sd, prefix):
 
 
 @torch.no_grad()
+def encode_test_image(cfg, B: int, seed: int) -> torch.Tensor:
+    """The encoder fixtures' input: a smooth image in [-1, 1] plus seeded texture (what `encode` sees: a normalised RGB
+    picture).  Fixtures too large to store it keep its sha256 instead (oracle/gen_golden.py run_vae_encode)."""
+    g = torch.Generator().manual_seed(seed)
+    S = cfg.image_size
+    yy, xx = torch.meshgrid(torch.linspace(-1, 1, S), torch.linspace(-1, 1, S), indexing="ij")
+    base = torch.stack([torch.sin(3 * xx + c) * torch.cos(2 * yy - c) for c in range(cfg.in_channels)], 0)
+    return (0.7 * base[None] + 0.3 * torch.randn(B, cfg.in_channels, S, S, generator=g)).clamp(-1, 1)
+
+
 def vae_decode(cfg, sd: Dict[str, torch.Tensor], z: torch.Tensor) -> torch.Tensor:
     """z: [B, embed_dim, h, w] (the sampler's latent) -> image [B, out_ch, h * 2^(levels-1), w * 2^(levels-1)]."""
     z = (1.0 / cfg.scale_factor) * z

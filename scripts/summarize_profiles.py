@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Turn the raw ncu outputs in gpurun_out/ into the small tracked summaries under profiles/.
+"""Turn the raw ncu outputs in profile_out/ into the small tracked summaries under profiles/.
 
     python scripts/summarize_profiles.py r1
 """
@@ -13,7 +13,7 @@ import sys
 from collections import defaultdict
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-OUT = os.path.join(ROOT, "gpurun_out")
+OUT = os.path.join(ROOT, "profile_out")
 PROF = os.path.join(ROOT, "profiles")
 
 KEYS = ["gpu__time_duration.sum", "dram__bytes_read.sum", "dram__bytes_write.sum", "gpu__dram_throughput.avg.pct_of_peak_sustained_elapsed",

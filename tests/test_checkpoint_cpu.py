@@ -1,15 +1,13 @@
 """Real-checkpoint path on the CPU (no GPU work: instantiation, key routing, config round trip, channel surgery)."""
-import importlib.util
 import os
 
 import pytest
 import torch
 
+from conftest import GOLD
 from gligen_b200 import checkpoint as CK
 from gligen_b200.pipeline import GROUNDING_INPUT, model_config
 from gligen_b200.spec import NAMED_CONFIGS, NAMED_VAE_CONFIGS, synthetic_state_dict, synthetic_vae_encoder_state_dict, synthetic_vae_state_dict
-
-REF = "/root/reference"
 
 
 def _config(name="tiny", vae="tiny_vae64"):
@@ -60,13 +58,10 @@ def test_inpaint_channel_surgery_matches_reference():
     CK.add_additional_channels(mine, 5)
     assert mine["input_blocks.0.0.weight"].shape == (320, 9, 3, 3) and torch.equal(mine["input_blocks.0.0.weight"][:, :4], w)
     assert mine["input_blocks.0.0.weight"][:, 4:].abs().sum() == 0 and torch.equal(mine["other"], torch.ones(2))
-    if os.path.isdir(REF):
-        spec = importlib.util.spec_from_file_location("_ref_convert_ckpt", os.path.join(REF, "convert_ckpt.py"))
-        ref = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(ref)
-        theirs = {"input_blocks.0.0.weight": w.clone(), "other": torch.ones(2)}
-        ref.add_additional_channels(theirs, 5)
-        assert torch.equal(theirs["input_blocks.0.0.weight"], mine["input_blocks.0.0.weight"])
+    # the reference's result on the same seeded weight (oracle/gen_golden_small.py)
+    gold = torch.load(os.path.join(GOLD, "reference_small.pt"))["add_additional_channels"]
+    assert torch.equal(gold["w"], w) and gold["num_additional_channels"] == 5
+    assert torch.equal(gold["out"], mine["input_blocks.0.0.weight"])
     # the widened tiny model loads into the inpainting variant
     from ldm.util import instantiate_from_config
     sd = synthetic_state_dict(NAMED_CONFIGS["tiny"], 0)

@@ -115,6 +115,7 @@ def test_vae_decoder_oracle_matches_reference(name, gold_file, tol):
         shapes = vae_decoder_param_shapes(cfg)
         assert len(shapes) == 140 and abs(sum(torch.Size(s).numel() for s in shapes.values()) - 49_490_199) == 0
         assert cfg.image_size == 512
-    img = VO.vae_decode(cfg, synthetic_vae_state_dict(cfg, 0), gold["z"])
+    st = gold.get("image_stride", 1)          # a full-size fixture keeps every st-th row and column of the reference image
+    img = VO.vae_decode(cfg, synthetic_vae_state_dict(cfg, 0), gold["z"])[..., ::st, ::st]
     assert img.shape == gold["image"].shape
     assert (img - gold["image"].float()).abs().max().item() <= tol * max(1.0, gold["image"].float().abs().max().item())

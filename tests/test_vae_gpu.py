@@ -1,6 +1,7 @@
 """VAE decoder on the GPU through the drop-in `ldm.models.autoencoder.AutoencoderKL.decode` against the REFERENCE decode
 goldens (same seeded weights and latents).  Tolerance: bf16 operands / fp32 accumulation through ~30 convolutions against an
 fp32 reference: rel-L2 <= 3e-2, max-abs <= 10 % of max|image| (measured values are printed)."""
+import hashlib
 import os
 
 import pytest
@@ -24,7 +25,8 @@ def test_vae_decode_matches_reference(name, B):
     m = m.to("cuda:0").eval()
     img = m.decode(gold["z"].to("cuda:0"))
     torch.cuda.synchronize()
-    r, mx = assert_close(img, gold["image"].float(), rel=3e-2, max_rel=0.10, what=f"{name} decode")
+    st = gold.get("image_stride", 1)          # a full-size fixture keeps every st-th row and column of the reference image
+    r, mx = assert_close(img[..., ::st, ::st], gold["image"].float(), rel=3e-2, max_rel=0.10, what=f"{name} decode")
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     m.decode(gold["z"].to("cuda:0"))
@@ -47,7 +49,14 @@ def test_vae_encode_matches_reference(name, B):
     sd.update(synthetic_vae_encoder_state_dict(cfg, 1))
     m.load_state_dict(sd, strict=True)
     m = m.to("cuda:0").eval()
-    x = gold["x"].float().to("cuda:0")
+    if "x" in gold:
+        x = gold["x"].float()
+    else:                                    # a full-size fixture stores the input's recipe and hash, not the image
+        from oracle import vae_oracle as VO
+        x = VO.encode_test_image(cfg, gold["B"], gold["seed"]).half()
+        assert hashlib.sha256(x.numpy().tobytes()).hexdigest() == gold["x_sha256"]
+        x = x.float()
+    x = x.to("cuda:0")
     mom = m.encode_moments(x)
     torch.cuda.synchronize()
     r, mx = assert_close(mom, gold["moments"], rel=3e-2, max_rel=0.10, what=f"{name} encode moments")
